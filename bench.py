@@ -13,10 +13,16 @@ EVERY step.  In the default (captured) mode the gradient all-reduce, the metric 
 libdmlb kernel (fused step exchange) and the optimizer is one more (K5 / K6).  Everything goes through the public API:
 TrainingPipeline.run() -> TrainValStage.train_epoch().
 
-Timing.  A timed WINDOW is exactly K steps bracketed by barrier + cuda synchronize on both sides, CUDA-event timed on the
-launching stream, max over ranks.  A single 20-step window of a 0.25 ms step is 5 ms long and one host hiccup doubles it
-(VERDICT r1), so windows are repeated — value and e2e windows alternating — until each arm has >= --min-seconds of timed
-region, and the MEDIAN window is reported (all window times are in the JSON).  `steps` stays K.
+Timing.  Each arm below times exactly K = --steps steps, split into windows of at least 20 steps (one window when K < 40);
+a window is one epoch with barrier + cuda synchronize around it, and CUDA events on the launching stream time its steps,
+from handing out the first batch to the end of the last step (max over ranks).  One host hiccup can double a 5 ms window
+(VERDICT r1), so value and e2e windows alternate and the MEDIAN time per step over the windows is reported (all window
+times are in the JSON).  The number of steps the model trains for depends on the arguments only.
+
+--dump-outputs DIR writes, after the timed steps, what the last step handed its caller (rank 0): the loss, the logits,
+the parameters and buffers after the optimizer step, and the reduced train metrics of the last window, as DIR/<name>.npy
+(float32; float64 for the buffers), at most 64 MB in all.  Such a run uses cuDNN's deterministic algorithms (as the MNIST
+CNN always does) instead of autotuned ones, so that two runs with the same arguments compute the same outputs.
 
   value   inputs already resident in HBM (K distinct batches), device-timed, max over ranks
   e2e     the same loop fed from pinned HOST memory: H2D copy of every batch; the step's reduced metrics land in mapped
@@ -43,6 +49,9 @@ from pathlib import Path
 ROOT = Path(__file__).resolve().parent
 if str(ROOT) not in sys.path:
     sys.path.insert(0, str(ROOT))
+# the tree may be read-only: no bytecode caches are written into it, by this process or the ones it spawns
+sys.dont_write_bytecode = True
+os.environ['PYTHONDONTWRITEBYTECODE'] = '1'
 
 WORKLOADS = {
     'mnist': {'metric': 'samples/sec (box, device-timed) MNIST CNN', 'batch': 32, 'shape': (1, 28, 28), 'classes': 10,
@@ -63,8 +72,8 @@ def parse_args():
     ap.add_argument('--warmup', type=int, default=20)
     ap.add_argument('--impl', choices=['native', 'reference'], default='native')
     ap.add_argument('--workload', choices=sorted(WORKLOADS), default='mnist')
-    ap.add_argument('--min-seconds', type=float, default=0.5, help='timed region per arm (windows are repeated)')
-    ap.add_argument('--max-windows', type=int, default=200)
+    ap.add_argument('--min-seconds', type=float, default=0.5,
+                    help='reference arm: timed region (windows of K steps are repeated)')
     ap.add_argument('--grad-wire', choices=['bf16', 'fp32'], default='bf16')
     ap.add_argument('--grad-route', choices=['auto', 'peer', 'nccl'], default='auto')
     ap.add_argument('--grad-algo', type=int, default=0, help='dmlb_comm_allreduce algo: 0 auto, 1 one-shot, 2 two-shot, 3 NVLS')
@@ -80,6 +89,7 @@ def parse_args():
                     help='BASELINE config 3: snapshot model/optimizer/tracker state after every window (= epoch)')
     ap.add_argument('--no-micro', action='store_true', help='skip the kernel / metric microbenchmarks')
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='native arm: write the last step\'s outputs as DIR/<name>.npy')
     args = ap.parse_args()
     args.channels_last = args.channels_last == 'on' or (args.channels_last == 'auto' and args.workload == 'resnet18')
     return args
@@ -189,7 +199,17 @@ def native_arm(args):
     eager_steps = 3 if args.workload == 'mnist' else 8  # (ResNet-18: the extra eager steps time DDP's rebuilt buckets)
     # graph mode spends the eager steps + 1 capture step before the first replay: keep all of that inside the warm-up
     K, W = args.steps, max(eager_steps + 5 if use_graph else 3, args.warmup)
-    torch.backends.cudnn.benchmark = True
+    plan = window_plan(K)
+    # cuDNN autotuning picks ResNet-18 convolutions 1.7 % faster than cuDNN's deterministic choice (B200, 1000 W).  On the
+    # MNIST CNN the step it leads to took 0.236-0.252 ms in 8 of 10 processes, against 0.231-0.233 ms in every process
+    # without it.  It may also pick other algorithms, hence other roundings, from run to run: runs whose outputs are
+    # compared do without it.
+    autotune = args.workload == 'resnet18' and not args.dump_outputs
+    torch.backends.cudnn.benchmark = autotune
+    torch.backends.cudnn.deterministic = not autotune
+
+    def per_step(window_ms):
+        return [ms / n for ms, n in zip(window_ms, plan)]
 
     def gen_batches(seed, count, pinned):
         g = torch.Generator().manual_seed(seed)
@@ -252,8 +272,6 @@ def native_arm(args):
             self.walls = {'value': [], 'e2e': []}
             self.launches = {'value': [], 'e2e': []}
             self.clocks = None
-            self.target = None  # number of window PAIRS, decided after the first pair
-            self.retries = 0
             self.host_reads = 0
             self.read_host = False
             self._older = None
@@ -269,15 +287,22 @@ def native_arm(args):
                 out = self.pipeline.models['net'](x)
             loss = self.loss(out.float(), y)
             self.track_reduce('accuracy', (out.argmax(1) == y).float().mean())
+            # in a captured step these are the graph's static outputs: every replay rewrites them
+            self.last_loss_logits = (loss.detach(), out.detach())
             return loss
 
         def table_columns(self):
             return [{'name': 'Epoch', 'metric': 'misc/epoch'}, {'name': 'Time/Epoch', 'metric': None},
                     {'name': 'Loss', 'metric': 'train/loss'}]
 
-        def feed(self, data):
+        def feed(self, data, events=None):
             """The 'DataLoader': hands out the next batch; in the e2e phase it first reads, on the host, the reduced
-            metrics of two steps ago out of the mapped result ring (what a progress bar would print)."""
+            metrics of two steps ago out of the mapped result ring (what a progress bar would print).  In a timed window
+            `events` bracket the steps themselves: the first is recorded before the first batch is handed out, the second
+            when the loop asks for a batch after the last step, so the epoch's set-up around them is not timed."""
+            if events is not None:
+                self.wall0 = time.perf_counter()
+                events[0].record()
             for batch in data:
                 if self.read_host:
                     if self._older is not None and 'train/loss' in self._older:
@@ -285,25 +310,28 @@ def native_arm(args):
                         self.host_reads += 1
                     self._older = self.live_metrics or None
                 yield batch
+            if events is not None:
+                events[1].record()
 
         def _window(self, kind):
-            data = (self.resident if kind == 'value' else self.host)[:K]
-            self.pipeline.datasets['train'] = self.feed(data)
+            i = len(self.windows[kind])
+            start = sum(plan[:i])
+            data = (self.resident if kind == 'value' else self.host)[start:start + plan[i]]
+            t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            self.pipeline.datasets['train'] = self.feed(data, (t0, t1))
             self.read_host, self._older = kind == 'e2e', None
-            sampler = ClockSampler(self.device.index) if (kind == 'value' and self.clocks is None) else None
+            # the polling thread takes the GIL from the host-bound step loop: it runs beside the first e2e window, not
+            # beside the headline arm (whose first window is its only one when K < 40)
+            sampler = ClockSampler(self.device.index) if (kind == 'e2e' and self.clocks is None) else None
             dist.barrier()
             torch.cuda.synchronize()
             if sampler:
                 sampler.start()
             n0 = N.launch_count()
             replays0 = self._graph.replays if self._graph is not None else 0
-            t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            wall0 = time.perf_counter()
-            t0.record()
-            self.train_epoch()  # <- the public per-step loop (stage.py train_epoch), exactly K steps
-            t1.record()
+            self.train_epoch()  # <- the public per-step loop (stage.py train_epoch) over this window's steps
             torch.cuda.synchronize()
-            wall = (time.perf_counter() - wall0) * 1e3
+            wall = (time.perf_counter() - self.wall0) * 1e3
             dist.barrier()
             if sampler:
                 self.clocks = sampler.stop()
@@ -331,23 +359,12 @@ def native_arm(args):
                     raise SystemExit('bench.py: the whole-step CUDA graph was not captured during the warm-up')
                 return
             self._window('value' if e % 2 == 1 else 'e2e')  # windows alternate so that drift hits both arms alike
-            pairs = len(self.windows['e2e'])
-            if e % 2 == 0:
-                if self.target is None and pairs >= 3:  # (median of three: one slow first window must not shorten the run)
-                    per_window = all_max(statistics.median(self.windows['value'] + self.windows['e2e'])) * 1e-3  # seconds
-                    self.target = int(min(args.max_windows, max(5, -(-args.min_seconds // max(per_window, 1e-6)))))
-                if self.target is not None and pairs >= self.target:
-                    v = statistics.median(self.windows['value'])
-                    x = statistics.median(self.windows['e2e'])
-                    # e2e does strictly more work than value: if it measures faster by > 2 % the windows are still too
-                    # noisy -> measure more (twice), then give up loudly
-                    bad = all_max(1 if x < 0.98 * v else 0)
-                    if bad and self.retries < 2:
-                        self.retries += 1
-                        self.target = pairs + self.target
-                    else:
-                        self.inconsistent = bool(bad)
-                        self.stop_stage()
+            if len(self.windows['e2e']) == len(plan):
+                v = statistics.median(per_step(self.windows['value']))
+                x = statistics.median(per_step(self.windows['e2e']))
+                # e2e does strictly more work than value: if it measures faster by > 2 % the windows were too noisy
+                self.inconsistent = bool(all_max(1 if x < 0.98 * v else 0))
+                self.stop_stage()
 
         def post_epoch(self):
             if args.checkpoint_every_epoch and self.pipeline.last_checkpoint_ms is not None:
@@ -389,6 +406,8 @@ def native_arm(args):
         raise SystemExit(f'bench.py: model replicas diverged across ranks: {digests}')
     if not all(torch.isfinite(flat.double().sum()).item() for _ in (0,)):
         raise SystemExit('bench.py: non-finite parameters after the run')
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, stage, pipeline)
 
     # ---- numbers ---------------------------------------------------------------------------------------------------------
     def gathered_windows(kind):
@@ -401,10 +420,10 @@ def native_arm(args):
     box = [None] * world
     dist.all_gather_object(box, stage.walls['e2e'])
     e2e_walls = [max(col) for col in zip(*box)]
-    value_ms = statistics.median(value_windows)
+    step_ms = statistics.median(per_step(value_windows))
     # host reads are part of e2e: per window the larger of the device time and the host wall time
-    e2e_ms = statistics.median([max(d, w) for d, w in zip(e2e_windows, e2e_walls)])
-    samples = K * BATCH * world
+    e2e_step_ms = statistics.median(per_step([max(d, w) for d, w in zip(e2e_windows, e2e_walls)]))
+    samples = BATCH * world  # per step
 
     # ---- in-situ gradient sync timing ----
     torch.cuda.synchronize()
@@ -447,8 +466,8 @@ def native_arm(args):
     live_cells = sum(m.lanes for m in graph.live_names.values()) if graph is not None and graph.live_names else \
         sum(m.lanes for m in pipeline.tracker.live_selection()[0].values())
     result = {
-        'metric': wl['metric'], 'value': round(samples / (value_ms * 1e-3), 1), 'unit': 'samples/s', 'n_gpus': world,
-        'steps': K, 'warmup': W, 'ms_per_step': round(value_ms / K, 4), 'higher_is_better': True, 'scaling': 'weak',
+        'metric': wl['metric'], 'value': round(samples / (step_ms * 1e-3), 1), 'unit': 'samples/s', 'n_gpus': world,
+        'steps': K, 'warmup': W, 'ms_per_step': round(step_ms, 4), 'higher_is_better': True, 'scaling': 'weak',
         'vs_baseline': None, 'dtype': 'bf16' if args.grad_wire == 'bf16' else 'f32', 'data': 'synthetic',
         'config': {'workload': wl['name'], 'global_batch': BATCH * world, 'parallelism': f'dp{world}',
                    'grad_wire': args.grad_wire, 'cuda_graph': bool(graph is not None),
@@ -464,23 +483,24 @@ def native_arm(args):
                    'python_gc': 'cyclic collector runs at epoch (= window) boundaries, not inside the step loop (stage.manual_gc)',
                    'metric_route': 'peer' if (pipeline.metric_comm is not None or graph is not None) else
                    ('single' if world == 1 else 'collective'),
-                   'timing': f'median of {len(value_windows)} windows of {K} steps per arm (value / e2e alternating), each '
-                             'bracketed by barrier + synchronize, CUDA events, max over ranks',
+                   'timing': f'{K} steps per arm in windows of {plan} steps (value / e2e alternating), median time per '
+                             'step over the windows; each window bracketed by barrier + synchronize, CUDA events, max '
+                             'over ranks',
                    'l2': ('K distinct batches; the MNIST working set (<10 MB) is L2-resident by the nature of the workload'
                           if args.workload == 'mnist' else
                           'K distinct batches of 38.5 MB each + 45 MB of gradients per step: larger than the 126 MB L2') +
                          '; the roofline microbench uses 1 GiB buffers'},
         'clocks': stage.clocks,
-        'e2e': {'value': round(samples / (e2e_ms * 1e-3), 1), 'unit': 'samples/s',
+        'e2e': {'value': round(samples / (e2e_step_ms * 1e-3), 1), 'unit': 'samples/s',
                 'h2d_bytes_per_step': BATCH * (4 * wl['shape'][0] * wl['shape'][1] * wl['shape'][2] + LABEL_BYTES),
                 'd2h_bytes_per_step': 12 + 9 * live_cells,  # stamp + status + {value, flag} per exchanged cell, written
-                'ms_per_step': round(e2e_ms / K, 4), 'host_reads': stage.host_reads,   # into mapped host memory
+                'ms_per_step': round(e2e_step_ms, 4), 'host_reads': stage.host_reads,   # into mapped host memory
                 'windows_ms': [round(w, 3) for w in e2e_windows]},
         'gpu_launches': int(statistics.median(stage.launches['value'])),
         'windows_ms': [round(w, 3) for w in value_windows],
-        'window_spread': {'min_ms': round(min(value_windows), 3), 'max_ms': round(max(value_windows), 3),
-                          'retries': stage.retries},
-        'wall_ms_per_step': round(statistics.median(stage.walls['value']) / K, 4),
+        'window_steps': plan,
+        'window_spread': {'min_ms': round(min(value_windows), 3), 'max_ms': round(max(value_windows), 3)},
+        'wall_ms_per_step': round(statistics.median(per_step(stage.walls['value'])), 4),
         'replicas_identical': replicas_identical,
         'roofline_in_situ': in_situ,
     }
@@ -488,7 +508,7 @@ def native_arm(args):
         result['ddp_buckets_in_situ'] = buckets_in_situ
     if args.checkpoint_every_epoch:
         ms = stage.checkpoint_ms
-        result['checkpoint'] = {'every': f'window of {K} steps (= one epoch)', 'snapshots': len(ms),
+        result['checkpoint'] = {'every': 'window (= one epoch)', 'snapshots': len(ms),
                                 'host_ms_per_epoch_median': round(statistics.median(ms), 3) if ms else None,
                                 'host_ms_per_epoch_max': round(max(ms), 3) if ms else None,
                                 'what': 'wall time the epoch loop spends on the snapshot (D2H into pinned staging is '
@@ -511,6 +531,41 @@ def native_arm(args):
     if pipeline.metric_comm is not None:
         pipeline.metric_comm.close()
     dist.destroy_process_group()
+
+
+def window_plan(k, min_steps=20):
+    """k timed steps as windows of at least `min_steps` steps each (one window when k < 2 * min_steps)."""
+    n = max(1, k // min_steps)
+    return [k // n + (i < k % n) for i in range(n)]
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(directory, stage, pipeline):
+    """What the last timed step handed its caller, as <directory>/<name>.npy: its loss and logits, the model's
+    parameters and buffers after the optimizer step, and the train metrics reduced over the last window."""
+    import numpy as np
+    import torch
+
+    torch.cuda.synchronize()
+    model = pipeline.models['net']
+    loss, logits = stage.last_loss_logits
+    with torch.no_grad():
+        arrays = {'loss': loss.float().cpu().numpy(), 'logits': logits.float().cpu().numpy(),
+                  'parameters': torch.cat([p.flatten().float() for p in model.parameters()]).cpu().numpy()}
+        buffers = [b.flatten().double() for b in model.buffers()]
+        if buffers:
+            arrays['buffers'] = torch.cat(buffers).cpu().numpy()
+        for name in ('train/loss', 'train/accuracy'):
+            arrays[name.replace('/', '_')] = torch.as_tensor(pipeline.tracker[name][-1]).float().cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise SystemExit(f'bench.py: the outputs take {total} bytes, more than --dump-outputs writes ({DUMP_BYTES})')
+    out = Path(directory)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out / f'{name}.npy', a)
 
 
 NVLINK_GBPS = 770.0  # measured per-direction peer bandwidth of this pool's B200s (B200_PROFILING.md; spec 900)
@@ -842,9 +897,9 @@ def _run_reference(world, steps, warmup, workload, min_seconds):
     if workload != 'mnist':
         raise SystemExit('bench.py: oracle/_ref (the installed reference) is needed for the ResNet-18 reference arm')
     cores = ref_port.usable_cores()
-    stock = ref_port.run_baseline(world=world, steps=max(steps, 200), warmup=max(3, warmup), total_threads=cores,
+    stock = ref_port.run_baseline(world=world, steps=steps, warmup=max(3, warmup), total_threads=cores,
                                   per_step_reduce=False)
-    strict = ref_port.run_baseline(world=world, steps=max(steps, 200), warmup=max(3, warmup), total_threads=cores,
+    strict = ref_port.run_baseline(world=world, steps=steps, warmup=max(3, warmup), total_threads=cores,
                                    per_step_reduce=True)
     stock.update({'kind': 'port', 'windows': 1, 'per_step_reduce_samples_per_s': strict['samples_per_s']})
     return stock

@@ -8,6 +8,8 @@ under oracle/shims/) on torch.distributed/gloo CPU and writes small fixtures to 
   grads_*.npz            per-rank local gradients (inputs) and the DDP(gloo)-reduced gradients (reference output)
   train_w{1,2,4,8}.json  a short TrainValStage + DDP(gloo) MNIST-CNN run on synthetic data: full tracker.histories
   train_clip_w{1,2}.json the same run with gradient_clip() != 0;  train_sched_w1.json with a StepLR scheduler
+  shard_fuzz.json        digests of util/data.py's answers to tests/test_shard_fuzz_vs_reference.py's random cases
+  metric_fuzz_w{1..4}.json  every rank's histories after tests/test_metric_fuzz_vs_reference.py's random sessions
 
 Usage (build container only):  python oracle/gen_golden.py
 Nothing on the GPU box may call this: /root/reference does not exist there; tests read the committed fixtures.
@@ -305,11 +307,63 @@ def gen_train():
         print(fname, {k: v[-1] for k, v in ranks[0]['histories'].items() if 'loss' in k})
 
 
+# ----------------------------------------------------------------------------------------------------------------------
+# 5. the reference's answers to the seeded random cases of the differential fuzz tests
+# ----------------------------------------------------------------------------------------------------------------------
+FUZZ_SEEDS = {1: range(60), 2: range(2000, 2012), 3: range(3000, 3012), 4: range(4000, 4010)}  # the tests' seeds
+
+
+def _fuzz_tests():
+    sys.path.insert(0, str(REPO / 'tests'))
+    import test_metric_fuzz_vs_reference
+    import test_shard_fuzz_vs_reference
+
+    return test_shard_fuzz_vs_reference, test_metric_fuzz_vs_reference
+
+
+def _fuzz_metrics_worker(rank, world, initfile, outdir, seeds):
+    _init(rank, world, initfile)
+    from dmlcloud.metrics import MetricTracker, Reduction
+
+    _, T = _fuzz_tests()
+    sessions = {}
+    for seed in seeds:
+        script = T.random_session(seed, world)
+        tracker = MetricTracker()
+        T.replay(tracker, Reduction, script, rank)
+        sessions[str(seed)] = {'script_sha256': T.script_digest(script), 'epoch': tracker.epoch,
+                               'histories': {k: [enc(v) for v in h] for k, h in tracker.histories.items()}}
+    Path(outdir, f'rank{rank}.json').write_text(json.dumps(sessions))
+    dist.destroy_process_group()
+
+
+def gen_fuzz():
+    from dmlcloud.util import data
+
+    S, _ = _fuzz_tests()
+    out = {'shard_indices': S.run_shard_indices(data.shard_indices),
+           'chunks_and_sequences': S.run_chunks_and_sequences(data.chunk_and_shard_indices, data.shard_sequence),
+           'dataset_epochs': S.run_dataset_epochs(data.ShardedSequenceDataset),
+           'interleave': S.run_interleave(data.interleave_batches)}
+    (GOLD / 'shard_fuzz.json').write_text(json.dumps(out))
+    print('shard_fuzz.json', {k: len(v) for k, v in out.items()})
+    for world, seeds in FUZZ_SEEDS.items():
+        out = _spawn(_fuzz_metrics_worker, world, list(seeds))
+        ranks = [json.loads((out / f'rank{r}.json').read_text()) for r in range(world)]
+        sessions = {}
+        for seed in map(str, seeds):
+            assert len({ranks[r][seed]['script_sha256'] for r in range(world)}) == 1
+            sessions[seed] = {'script_sha256': ranks[0][seed]['script_sha256'],
+                              'ranks': [{k: ranks[r][seed][k] for k in ('epoch', 'histories')} for r in range(world)]}
+        (GOLD / f'metric_fuzz_w{world}.json').write_text(json.dumps({'world': world, 'sessions': sessions}))
+        print(f'metric_fuzz_w{world}.json', len(sessions), 'sessions')
+
+
 if __name__ == '__main__':
     if not Path('/root/reference/dmlcloud').is_dir():
         sys.exit('gen_golden.py needs /root/reference (build container only)')
     GOLD.mkdir(parents=True, exist_ok=True)
-    which = sys.argv[1:] or ['shards', 'metrics', 'grads', 'train']
+    which = sys.argv[1:] or ['shards', 'metrics', 'grads', 'train', 'fuzz']
     if 'shards' in which:
         gen_shards()
     if 'metrics' in which:
@@ -318,3 +372,5 @@ if __name__ == '__main__':
         gen_grads()
     if 'train' in which:
         gen_train()
+    if 'fuzz' in which:
+        gen_fuzz()

@@ -1,7 +1,8 @@
 """The differential fuzz of tests/test_metric_fuzz_vs_reference.py with the PRODUCT in the loop: libdmlb's device slab (K3 fold,
-K4 reduce / peer exchange) replays the same seeded random sessions as the installed, unmodified reference (oracle/_ref travels
-to the GPU box) and must agree with it within SURVEY §8d's tolerances — and with the slab oracle bit for bit.  World size 2
-and 4 run as separate processes sharing the GPU (CUDA-IPC peer mappings, or real NVLink peers on a multi-GPU box)."""
+K4 reduce / peer exchange) replays the same seeded random sessions the unmodified reference replayed (its answers are stored
+in tests/golden/metric_fuzz_w*.json) and must agree with it within SURVEY §8d's tolerances — and with the slab oracle bit
+for bit.  World size 2 and 4 run as separate processes sharing the GPU (CUDA-IPC peer mappings, or real NVLink peers on a
+multi-GPU box)."""
 import json
 from pathlib import Path
 
@@ -9,9 +10,9 @@ import pytest
 import torch
 
 from helpers import init_gloo, rank_device, spawn
-from test_metric_fuzz_vs_reference import REF_METRICS, run_seeds
+from test_metric_fuzz_vs_reference import run_seeds
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not REF_METRICS.exists(), reason='oracle/_ref not built')]
+pytestmark = pytest.mark.gpu
 
 
 def test_random_sessions_on_the_device_slab_match_reference_and_oracle_w1():

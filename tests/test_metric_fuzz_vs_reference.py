@@ -1,37 +1,54 @@
-"""Differential fuzz of the metric path (SURVEY §8 a-4..a-8) against the INSTALLED, unmodified reference.
+"""Differential fuzz of the metric path (SURVEY §8 a-4..a-8) against the unmodified reference.
 
-`oracle/_ref` (pip install --target of the reference, oracle/Makefile) holds the reference's own `dmlcloud/metrics.py`; it
-needs nothing but torch, so it is loaded by path here.  Seeded random sessions — random metric sets (all reductions, `dim`
-subsets, int64 and fp32 values, rank-local metrics, un-reduced metrics), random step counts, epochs in which a metric gets no
-value, late registration, prefix reduces — are replayed on the reference's MetricTracker and on this repo's MetricTracker
-(host logic) over oracle/slab_oracle.py (the bit-level restatement of the device slab the GPU tests compare libdmlb with),
-at world size 1 and 2 (gloo).  This pins host logic + slab oracle to the reference far beyond the fixed golden sessions:
-the GPU parity tests then carry that over to the kernels.
+Seeded random sessions — random metric sets (all reductions, `dim` subsets, int64 and fp32 values, rank-local metrics,
+un-reduced metrics), random step counts, epochs in which a metric gets no value, late registration, prefix reduces — are
+replayed on this repo's MetricTracker (host logic) over oracle/slab_oracle.py (the bit-level restatement of the device slab
+the GPU tests compare libdmlb with), at world size 1, 2 and 3 (gloo), and compared with what the reference's own
+MetricTracker computed for the same sessions: oracle/gen_golden.py replayed them on the reference and stored every rank's
+resulting histories in tests/golden/metric_fuzz_w{1,2,3,4}.json (the script's SHA-256 beside them pins the session).
+This pins host logic + slab oracle to the reference far beyond the fixed golden sessions: the GPU parity tests then carry
+that over to the kernels.
 
 Tolerances (SURVEY §8d): MIN / MAX, integer results, None patterns, dtypes, shapes, epochs: exact; fp32 MEAN / SUM: rtol 1e-5,
 atol 1e-6 (the reference reduces a stacked fp32 tensor, the slab accumulates in fp64 and rounds once).
 """
-import importlib.util
+import functools
+import hashlib
 import json
 from pathlib import Path
+from types import SimpleNamespace
 
 import numpy as np
 import pytest
 import torch
 
-from helpers import REPO, init_gloo, spawn
-
-REF_METRICS = REPO / 'oracle' / '_ref' / 'dmlcloud' / 'metrics.py'
-pytestmark = pytest.mark.skipif(not REF_METRICS.exists(), reason='oracle/_ref not built (make -C oracle _ref)')
+from conftest import decode_entry, load_json
+from helpers import init_gloo, spawn
 
 REDUCTIONS = ('MEAN', 'SUM', 'MIN', 'MAX')
 
 
-def load_reference_metrics():
-    spec = importlib.util.spec_from_file_location('_installed_reference_metrics', REF_METRICS)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
+def script_digest(script):
+    return hashlib.sha256(json.dumps(script).encode()).hexdigest()
+
+
+@functools.lru_cache(maxsize=None)
+def reference_sessions(world):
+    return load_json(f'metric_fuzz_w{world}.json')['sessions']
+
+
+def reference_tracker(world, seed, rank, script):
+    """The reference MetricTracker's state after `script` on `rank`, as stored by oracle/gen_golden.py."""
+    session = reference_sessions(world)[str(seed)]
+    assert session['script_sha256'] == script_digest(script), ('the session generator changed', world, seed)
+    state = session['ranks'][rank]
+
+    def decode(e):
+        v = decode_entry(e)
+        return torch.from_numpy(v) if isinstance(v, np.ndarray) else v
+
+    return SimpleNamespace(epoch=state['epoch'],
+                           histories={name: [decode(e) for e in h] for name, h in state['histories'].items()})
 
 
 def random_session(seed, world):
@@ -118,17 +135,15 @@ def compare(want_tracker, got_tracker, script, seed, exact=False):
 
 def run_seeds(seeds, world, rank, device=None, comm=None):
     """device=None: this repo's MetricTracker over the slab oracle (CPU).  device=cuda: the product — libdmlb's device slab
-    (and `comm`, the peer communicator, at world > 1) — checked against the installed reference AND, bit for bit, against
-    the slab oracle."""
+    (and `comm`, the peer communicator, at world > 1) — checked against the reference AND, bit for bit, against the slab
+    oracle."""
     from dmlcloud_b200.metrics import MetricTracker, Reduction
     from oracle.slab_oracle import OracleSlab
 
-    ref = load_reference_metrics()
     checked = 0
     for seed in seeds:
         script = random_session(seed, world)
-        want = ref.MetricTracker()
-        replay(want, ref.Reduction, script, rank)
+        want = reference_tracker(world, seed, rank, script)
         restated = MetricTracker()
         restated.bind(slab=OracleSlab())
         replay(restated, Reduction, script, rank)
